@@ -5,7 +5,7 @@ One "step" = one complete pass of the hot path over one batch: the infer branch 
 conditioner (start state, all sampler steps through DiffNet, denorm epilogue) for B utterances of T frames.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--config 1|2|3|4|sweep] [--precision fp16s|fp16x2|fp16x3|fp16|fp32]
-                  [--impl reference]
+                  [--impl reference] [--dump-outputs DIR]
 
 --config (BASELINE.json `configs`, default 2 = the configuration the metric is quoted on):
    1  DiffSpeech LJ   B=1  T=512   K=100  DDPM              (the reference's own CPU-runnable case)
@@ -404,7 +404,7 @@ def timed_steps(arm, steps, warmup, world, dev, flush, gather_total=None, clocks
     if world > 1:
         dist.all_reduce(total_ms, op=dist.ReduceOp.MAX)
     assert torch.isfinite(mel).all()
-    return float(total_ms.item()), (l1 - l0), clk
+    return float(total_ms.item()), (l1 - l0), clk, mel
 
 
 def roofline_of(arm, prec, ms_per_step):
@@ -489,13 +489,14 @@ def e2e_of(dsx, cfg, prec, dev, rank, world, steps):
             "api": "dsx_infer_host (C ABI, pinned host buffers)"}
 
 
-def bench_config(dsx, cfg, prec, args, dev, rank, world, local_rank, flush, full=True):
+def bench_config(dsx, cfg, prec, args, dev, rank, world, local_rank, flush, full=True, keep_output=False):
     arm = Arm(dsx, cfg, prec, dev, rank)
     B, T = arm.B, arm.T
-    total_ms, launches, clk = timed_steps(arm, args.steps, args.warmup, world, dev, flush, gather_total=B * world,
-                                          clocks_index=local_rank)
+    total_ms, launches, clk, mel = timed_steps(arm, args.steps, args.warmup, world, dev, flush, gather_total=B * world,
+                                               clocks_index=local_rank)
     ms = total_ms / args.steps
     out = {"value": world * B * T / (ms * 1e-3), "ms_per_step": ms, "launches": int(launches), "clocks": clk,
+           "mel": mel.cpu() if keep_output else None,
            "roofline": roofline_of(arm, prec, ms) if prec != "fp32" else None,
            "workspace_bytes": arm.s.info(arm.capi.INFO_WORKSPACE_BYTES)}
     arm.close()
@@ -516,7 +517,13 @@ def main():
     ap.add_argument("--cpu-evals", type=int, default=3)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the mel of the last timed step (what the caller receives, [B, T, 80]) as DIR/mel.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the dsx arm; the reference arm only times the CPU path")
 
     # stdout carries exactly ONE JSON line: everything libraries print there (NCCL's version banner, ...) goes to stderr
     global _JSON_OUT
@@ -543,8 +550,13 @@ def main():
 
     prec = args.precision
     flush = torch.empty(256 * 1024 * 1024 // 4, device=dev)       # > 126 MB L2
-    main_res = bench_config(dsx, cfg, prec, args, dev, rank, world, local_rank, flush)
+    main_res = bench_config(dsx, cfg, prec, args, dev, rank, world, local_rank, flush, keep_output=bool(args.dump_outputs))
     B, T, K = cfg["B"], cfg["T"], cfg["K"]
+    if args.dump_outputs and rank == 0:
+        # inputs, weights and noise seeds depend on the arguments alone, so two builds run with the same arguments can be
+        # compared output for output
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "mel.npy"), main_res.pop("mel").numpy().astype(np.float32))
 
     extra = {}
     if not args.no_extra and world == 1 and args.config != "sweep":
@@ -552,14 +564,14 @@ def main():
             if other == prec:
                 continue
             arm = Arm(dsx, cfg, other, dev, rank)
-            tms, _, _ = timed_steps(arm, 2, 2, world, dev, flush)
+            tms, _, _, _ = timed_steps(arm, 2, 2, world, dev, flush)
             arm.close()
             extra[other] = {"value": B * T / (tms / 2 * 1e-3), "unit": "frames/s", "ms_per_step": tms / 2, "note": NOTES[other]}
     if not args.no_extra and world > 1 and 32 % world == 0:
         # BASELINE configs[3] strong-scaled: B = 32 utterances in total, 32 / N per GPU, one all-gather per step
         c4 = CONFIGS["4"]
         arm = Arm(dsx, c4, prec, dev, rank, B=32 // world)
-        tms, _, _ = timed_steps(arm, 2, 2, world, dev, flush, gather_total=32)
+        tms, _, _, _ = timed_steps(arm, 2, 2, world, dev, flush, gather_total=32)
         arm.close()
         extra["strong_config4"] = {"value": 32 * c4["T"] / (tms / 2 * 1e-3), "unit": "frames/s", "ms_per_step": tms / 2, "scaling": "strong",
                                    "workload": c4["name"], "B_total": 32, "B_per_gpu": 32 // world,

@@ -10,3 +10,7 @@ Parity pinning: the reference has no tests or golden vectors for this path
 imported from /root/reference in the build container (``oracle/ref_bridge.py`` +
 ``oracle/gen_golden.py``); the vectors it produced are committed in ``tests/golden``.
 """
+
+# ATen's CPU convolutions split their float32 sums by the number of intra-op threads: the golden vectors are recorded, and
+# must be compared bit for bit, at this count
+FIXTURE_THREADS = 8

@@ -18,6 +18,7 @@ from collections import deque
 import numpy as np
 import torch
 
+from . import FIXTURE_THREADS
 from . import diffnet_oracle as O
 from . import ref_bridge
 
@@ -56,7 +57,7 @@ def make_ref_gd(ns, net, betas, K_step):
 
 def main():
     assert ref_bridge.available(), "needs /root/reference"
-    torch.set_num_threads(8)
+    torch.set_num_threads(FIXTURE_THREADS)
     ns = ref_bridge.load("usr/configs/lj_ds_beta6.yaml")
     sdt = ns.sdt
     os.makedirs(OUT, exist_ok=True)

@@ -1,5 +1,5 @@
 """TEST INFRASTRUCTURE ONLY -- pins oracle/hifigan_oracle.py to the LIVE reference (container only: needs /root/reference)
-and writes tests/golden/hifigan_nsf.npz.  Run:  python oracle/gen_golden_hifigan.py
+and writes tests/golden/hifigan_nsf.npz and hifigan_nsf_B1T9.npz.  Run:  python oracle/gen_golden_hifigan.py
 
 The reference module is imported unmodified (stubs only for librosa / pycwt and scipy.signal.kaiser, which newer SciPy moved
 to scipy.signal.windows); weights are the constructor's random initialisation under a fixed seed, inputs are seeded; the NSF
@@ -13,7 +13,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-from oracle import hifigan_oracle as H  # noqa: E402
+from oracle import FIXTURE_THREADS, hifigan_oracle as H  # noqa: E402
 
 REF_ROOT = os.environ.get("DSX_REFERENCE_ROOT", "/root/reference")
 
@@ -34,6 +34,7 @@ def load_reference():
 
 def make_case(seed=0, B=2, T=16):
     HifiGanGenerator = load_reference()
+    torch.set_num_threads(FIXTURE_THREADS)
     h = dict(H.HPARAMS_TTS, upsample_initial_channel=32)     # the shipped topology at 1/4 of the width: a 250 KB fixture
     torch.manual_seed(seed)
     g = HifiGanGenerator(h).eval()
@@ -45,7 +46,24 @@ def make_case(seed=0, B=2, T=16):
     return g, h, sd, mel, f0
 
 
+def write_odd_length_case():
+    """One utterance of odd length (T = 9) through the weights of the main fixture (weight seed 0), the NSF source's random
+    draws under seed 11: tests/golden/hifigan_nsf_B1T9.npz (inputs and output only; the weights are in hifigan_nsf.npz)."""
+    g, h, sd, _, _ = make_case(seed=0)
+    _, _, _, mel, f0 = make_case(seed=3, B=1, T=9)
+    with torch.no_grad():
+        torch.manual_seed(11)
+        ref = g(mel, f0)
+        torch.manual_seed(11)
+        ora = H.generator(sd, h, mel, f0)
+    assert torch.equal(ref, ora), "the oracle must be bit-exact against the reference"
+    out = os.path.join(ROOT, "tests", "golden", "hifigan_nsf_B1T9.npz")
+    np.savez_compressed(out, mel=mel.numpy(), f0=f0.numpy(), wav_nsf=ref.numpy(), rng_seed=np.int64(11))
+    print("wrote", out)
+
+
 def main():
+    write_odd_length_case()
     g, h, sd, mel, f0 = make_case()
     with torch.no_grad():
         torch.manual_seed(7)

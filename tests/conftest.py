@@ -28,6 +28,16 @@ HP = dict(hidden_size=256, residual_layers=20, residual_channels=256, dilation_c
           audio_num_mel_bins=80, keep_bins=80, schedule_type="linear", max_beta=0.06, timesteps=100, K_step=100)
 
 
+@pytest.fixture
+def fixture_threads():
+    """The CPU oracle agrees bit for bit with the golden vectors at the intra-op thread count they were recorded with."""
+    from oracle import FIXTURE_THREADS
+    n = torch.get_num_threads()
+    torch.set_num_threads(FIXTURE_THREADS)
+    yield
+    torch.set_num_threads(n)
+
+
 @pytest.fixture(scope="session")
 def lib_built():
     import __graft_entry__

@@ -1,7 +1,7 @@
 """The INSTALLED drop-in subclasses, end to end on the GPU (VERDICT r01 item 5): a stand-in reference tree
 (tests/standin_ref.py: the reference's module paths / class names / constructors, none of its sampling code) is written to a
 temp directory, `dropin.install()` patches it exactly as it patches the live tree (tests/test_reference_live.py checks that
-side in the build container), models are built the way the task files build them, and `forward(infer=True)` of each of
+side against a fixture recorded from the reference), models are built the way the task files build them, and `forward(infer=True)` of each of
 the three sampler classes is compared with the live reference's golden output."""
 import os
 import subprocess

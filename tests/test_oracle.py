@@ -7,6 +7,8 @@ import torch
 from conftest import golden, rs_normal
 from oracle import diffnet_oracle as O
 
+pytestmark = pytest.mark.usefixtures("fixture_threads")
+
 
 def test_schedules_match_reference_buffers():
     g = golden("schedules.npz")
