@@ -9,7 +9,8 @@ import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 SRC = [os.path.join(HERE, "csrc", f) for f in ("dsx_api.cu", "dsx_simt.cu", "dsx_tc.cu", "dsx_stack.cu", "dsx_selftest.cu")]
-HDR = [os.path.join(HERE, "csrc", f) for f in ("dsx_internal.h", "dsx_ptx.cuh", "dsx_rng.cuh", "dsx_tc_common.cuh")] + \
+HDR = [os.path.join(HERE, "csrc", f) for f in ("dsx_internal.h", "dsx_ptx.cuh", "dsx_rng.cuh", "dsx_tc_common.cuh",
+                                                  "dsx_update.cuh")] + \
       [os.path.join(os.path.dirname(HERE), "include", "dsx.h")]
 LIB = os.path.join(HERE, "lib", "libdsx.so")
 NVCC_FLAGS = ["-std=c++17", "-O3", "-lineinfo", "-gencode", "arch=compute_100a,code=sm_100a",

@@ -122,64 +122,92 @@ void reset_flags(dsx_handle* h) {
   h->flags_kind = 0;
 }
 
-// Residual layers [0, nl) of one evaluation; `head` (may be null): what follows them in the step.  Returns through
-// *head_done whether the head ran inside the stack launch (the caller then skips launch_tc_head).
-static int run_layers(dsx_handle* h, const Geom& g, int row0, int row_per_b, int nl, cudaStream_t s, const HeadArgs* head = nullptr,
-                      bool* head_done = nullptr) {
-  if (head_done) *head_done = false;
-  const bool tc = h->precision != DSX_PREC_FP32_SIMT;
-  cudaEvent_t e0 = nullptr, e1 = nullptr;
-  if (h->profile == 1) {
-    while (h->prof_events.size() < h->prof_used + 2) {
-      cudaEvent_t e;
-      DSX_CUDA(cudaEventCreate(&e));
-      h->prof_events.push_back(e);
-    }
-    e0 = h->prof_events[h->prof_used];
-    e1 = h->prof_events[h->prof_used + 1];
-    h->prof_used += 2;
-    DSX_CUDA(cudaEventRecord(e0, s));
+// DSX_OPT_PROFILE: when `mode` is the selected one, record the start of a (start, stop) pair of CUDA events; *stop is the
+// event the caller records to end it (null otherwise).
+static int prof_start(dsx_handle* h, int mode, cudaStream_t s, cudaEvent_t* stop) {
+  *stop = nullptr;
+  if (h->profile != mode) return DSX_OK;
+  while (h->prof_events.size() < h->prof_used + 2) {
+    cudaEvent_t e;
+    DSX_CUDA(cudaEventCreate(&e));
+    h->prof_events.push_back(e);
   }
-  if (tc) {
-    // weight set of DSX_PREC_FP16S: evaluation (= table row) j of a loop uses set j % R
-    if (tc_stack_usable(h, g)) {
-      const bool fuse = head && head->flags && h->fused_head && nl == h->m.L && h->profile != 2;
-      DSX_TRY(launch_tc_stack(h, nl, g, row0, row_per_b, row0, s, fuse ? head : nullptr));
-      if (fuse && head_done) *head_done = true;
-    } else {
-      DSX_TRY(launch_tc_layers(h, 0, nl, g, row0, row_per_b, s));
-    }
-  } else {
-    for (int l = 0; l < nl; ++l) DSX_TRY(launch_simt_layer(h, l, g, row0, row_per_b, s));
-  }
-  if (h->profile == 1) DSX_CUDA(cudaEventRecord(e1, s));
+  *stop = h->prof_events[h->prof_used + 1];
+  DSX_CUDA(cudaEventRecord(h->prof_events[h->prof_used], s));
+  h->prof_used += 2;
   return DSX_OK;
 }
 
-// One DiffNet evaluation: x (any strides) -> eps (contiguous [B,1,M,T]).
+static dsx_strides contiguous_mel(int M, int T) {
+  dsx_strides xs;
+  xs.b = static_cast<int64_t>(M) * T;
+  xs.c = T;
+  xs.t = 1;
+  return xs;
+}
+
+// The head of DSX_PREC_FP32_SIMT as CUDA-core launches, the flags read as by k_tc_head.  eps goes to ha.eps, else to the
+// history slot of the PNDM step, else to scratch slot 4 of ws.EPS.
+static int simt_head(dsx_handle* h, const Geom& g, const HeadArgs& ha, cudaStream_t s) {
+  const size_t mel = static_cast<size_t>(g.B) * h->m.M * g.T;
+  const PlmsFuse* pl = ha.plms;
+  float* eps = ha.eps ? ha.eps : (pl && pl->eps_store) ? pl->eps_store : h->ws.EPS + 4 * mel;
+  float* x = ha.x;
+  dsx_strides xs = ha.xs;
+  if (ha.flags & TC_HEAD) DSX_TRY(launch_head(h, g, eps, s));
+  if (ha.flags & TC_UPDATE) DSX_TRY(launch_ddpm_update(h, x, eps, ha.noise, ha.seed, ha.offset, ha.c, mel, g.T, s));
+  if (ha.flags & TC_PLMS) {
+    if (pl->x_out) { x = pl->x_out; xs = contiguous_mel(h->m.M, g.T); }
+    DSX_TRY(launch_plms_update(h, x, ha.x, eps, pl->h1, pl->h2, pl->h3, pl->c, mel, s));
+  }
+  if (ha.flags & TC_INPROJ) DSX_TRY(launch_inproj(h, x, xs, g, s));
+  return DSX_OK;
+}
+
+// Input projection of a call's first evaluation (table row (row0, row_per_b)); every later one runs in the head of the
+// evaluation before it (TC_INPROJ).
+static int start_eval(dsx_handle* h, const Geom& g, float* x, dsx_strides xs, int row0, int row_per_b, cudaStream_t s) {
+  if (h->precision == DSX_PREC_FP32_SIMT) return launch_inproj(h, x, xs, g, s);
+  HeadArgs ha;
+  ha.flags = TC_INPROJ; ha.x = x; ha.xs = xs; ha.next_row0 = row0; ha.row_per_b = row_per_b;
+  return launch_tc_head(h, g, ha, s);
+}
+
+// One evaluation: residual layers [0, nl) of table row (row0, row_per_b), then the head `ha` describes (none when ha.flags
+// is 0).  The stack kernel runs both in one launch where it can take the call; otherwise the head is a launch of its own:
+// k_tc_head, or the CUDA-core kernels of DSX_PREC_FP32_SIMT.  Weight set of DSX_PREC_FP16S: row j of a loop uses set j % R.
+static int run_step(dsx_handle* h, const Geom& g, int row0, int row_per_b, int nl, const HeadArgs& ha, cudaStream_t s) {
+  const bool fp32 = h->precision == DSX_PREC_FP32_SIMT;
+  bool fused = false;
+  cudaEvent_t stop;
+  DSX_TRY(prof_start(h, 1, s, &stop));     // DSX_OPT_PROFILE = 1: one bracket per evaluation, around the residual stack
+  if (fp32) {
+    for (int l = 0; l < nl; ++l) DSX_TRY(launch_simt_layer(h, l, g, row0, row_per_b, s));
+  } else if (tc_stack_usable(h, g)) {
+    fused = ha.flags && h->fused_head && nl == h->m.L && h->profile != 2;
+    DSX_TRY(launch_tc_stack(h, nl, g, row0, row_per_b, row0, s, fused ? &ha : nullptr));
+  } else {
+    DSX_TRY(launch_tc_layers(h, 0, nl, g, row0, row_per_b, s));
+  }
+  if (stop) DSX_CUDA(cudaEventRecord(stop, s));
+  if (!ha.flags || fused) return DSX_OK;
+  DSX_TRY(prof_start(h, 2, s, &stop));     // DSX_OPT_PROFILE = 2: around the separate head
+  DSX_TRY(fp32 ? simt_head(h, g, ha, s) : launch_tc_head(h, g, ha, s));
+  if (stop) DSX_CUDA(cudaEventRecord(stop, s));
+  return DSX_OK;
+}
+
+// One DiffNet evaluation: x (any strides) -> eps (contiguous [B,1,M,T]).  Under dsx_debug_set_layer_limit only the first
+// layers run, and no head.
 static int run_eval(dsx_handle* h, const float* x, dsx_strides xs, const Geom& g, int row0, int row_per_b, float* eps,
                     cudaStream_t s) {
-  const bool tc = h->precision != DSX_PREC_FP32_SIMT;
   const int nl = (h->layer_limit >= 0) ? std::min(h->layer_limit, h->m.L) : h->m.L;
-  const DdpmCoef none{};
-  if (tc)
-    DSX_TRY(launch_tc_head(h, g, TC_INPROJ, const_cast<float*>(x), xs, nullptr, nullptr, 0, 0, none, row0, row_per_b, s));
-  else
-    DSX_TRY(launch_inproj(h, x, xs, g, row0, row_per_b, s));
   HeadArgs ha;
-  ha.flags = TC_HEAD | TC_WRITE_EPS;
+  ha.flags = nl == h->m.L ? TC_HEAD | TC_WRITE_EPS : 0;
   ha.x = const_cast<float*>(x);          // (read only with these flags)
-  ha.xs = xs;
-  ha.eps = eps;
-  bool head_done = false;
-  DSX_TRY(run_layers(h, g, row0, row_per_b, nl, s, (tc && nl == h->m.L) ? &ha : nullptr, &head_done));
-  if (nl == h->m.L && !head_done) {
-    if (tc)
-      DSX_TRY(launch_tc_head(h, g, TC_HEAD | TC_WRITE_EPS, nullptr, xs, eps, nullptr, 0, 0, none, row0, row_per_b, s));
-    else
-      DSX_TRY(launch_head(h, g, eps, s));
-  }
-  return DSX_OK;
+  ha.xs = xs; ha.eps = eps;
+  DSX_TRY(start_eval(h, g, ha.x, xs, row0, row_per_b, s));
+  return run_step(h, g, row0, row_per_b, nl, ha, s);
 }
 
 // Workspace + tensor maps for (B, T) and, when `cond` is given, the conditioner pack and its hoisted projection (the
@@ -207,14 +235,6 @@ static int prepare(dsx_handle* h, const float* cond, dsx_strides cs, int B, int 
   return DSX_OK;
 }
 
-static dsx_strides contiguous_mel(int M, int T) {
-  dsx_strides xs;
-  xs.b = static_cast<int64_t>(M) * T;
-  xs.c = T;
-  xs.t = 1;
-  return xs;
-}
-
 static int sample_ddpm_impl(dsx_handle* h, float* x, const Geom& g, int t_start, int n_steps, const float* noise,
                             uint64_t seed, cudaStream_t s) {
   const size_t mel = static_cast<size_t>(g.B) * h->m.M * g.T;
@@ -224,44 +244,19 @@ static int sample_ddpm_impl(dsx_handle* h, float* x, const Geom& g, int t_start,
   DSX_CUDA(cudaStreamSynchronize(s));   // tv is a stack-owned staging buffer
   DSX_TRY(launch_embed_table(h, h->ws.TVALS, n_steps, s));
   const dsx_strides xs = contiguous_mel(h->m.M, g.T);
-  const bool tc = h->precision != DSX_PREC_FP32_SIMT;
-  if (tc) DSX_TRY(launch_tc_head(h, g, TC_INPROJ, x, xs, nullptr, nullptr, 0, 0, DdpmCoef{}, 0, 0, s));
+  DSX_TRY(start_eval(h, g, x, xs, 0, 0, s));
   for (int j = 0; j < n_steps; ++j) {
     const int t = t_start - 1 - j;
-    if (!tc) DSX_TRY(run_eval(h, x, xs, g, j, 0, h->ws.EPS, s));
-    DdpmCoef c;
-    c.A = h->sched[DSX_SCH_SQRT_RECIP_ALPHAS_CUMPROD][t];
-    c.Bc = h->sched[DSX_SCH_SQRT_RECIPM1_ALPHAS_CUMPROD][t];
-    c.c1 = h->sched[DSX_SCH_POSTERIOR_MEAN_COEF1][t];
-    c.c2 = h->sched[DSX_SCH_POSTERIOR_MEAN_COEF2][t];
-    c.sigma = (t == 0) ? 0.f : expf(0.5f * h->sched[DSX_SCH_POSTERIOR_LOG_VARIANCE_CLIPPED][t]);
-    const float* nz = noise ? noise + static_cast<size_t>(j) * mel : nullptr;
-    if (tc) {
-      // 20 fused residual-layer kernels, then ONE kernel: head GEMMs + p_sample update + next step's input projection
-      const int flags = TC_HEAD | TC_UPDATE | (j + 1 < n_steps ? TC_INPROJ : 0);
-      HeadArgs ha;
-      ha.flags = flags; ha.x = x; ha.xs = xs; ha.noise = nz; ha.seed = seed; ha.offset = static_cast<uint64_t>(j); ha.c = c;
-      ha.next_row0 = j + 1; ha.row_per_b = 0;
-      bool head_done = false;
-      DSX_TRY(run_layers(h, g, j, 0, h->m.L, s, &ha, &head_done));
-      if (head_done) continue;               // ONE launch did the whole diffusion step
-      cudaEvent_t e0 = nullptr, e1 = nullptr;
-      if (h->profile == 2) {                       // DSX_OPT_PROFILE = 2: bracket the head kernel instead of the layer stack
-        while (h->prof_events.size() < h->prof_used + 2) {
-          cudaEvent_t e;
-          DSX_CUDA(cudaEventCreate(&e));
-          h->prof_events.push_back(e);
-        }
-        e0 = h->prof_events[h->prof_used];
-        e1 = h->prof_events[h->prof_used + 1];
-        h->prof_used += 2;
-        DSX_CUDA(cudaEventRecord(e0, s));
-      }
-      DSX_TRY(launch_tc_head(h, g, flags, x, xs, nullptr, nz, seed, static_cast<uint64_t>(j), c, j + 1, 0, s));
-      if (e1) DSX_CUDA(cudaEventRecord(e1, s));
-    } else {
-      DSX_TRY(launch_ddpm_update(h, x, h->ws.EPS, nz, seed, static_cast<uint64_t>(j), c, mel, g.T, s));
-    }
+    HeadArgs ha;
+    ha.flags = TC_HEAD | TC_UPDATE | (j + 1 < n_steps ? TC_INPROJ : 0);
+    ha.x = x; ha.xs = xs; ha.seed = seed; ha.offset = static_cast<uint64_t>(j); ha.next_row0 = j + 1;
+    ha.noise = noise ? noise + static_cast<size_t>(j) * mel : nullptr;
+    ha.c.A = h->sched[DSX_SCH_SQRT_RECIP_ALPHAS_CUMPROD][t];
+    ha.c.Bc = h->sched[DSX_SCH_SQRT_RECIPM1_ALPHAS_CUMPROD][t];
+    ha.c.c1 = h->sched[DSX_SCH_POSTERIOR_MEAN_COEF1][t];
+    ha.c.c2 = h->sched[DSX_SCH_POSTERIOR_MEAN_COEF2][t];
+    ha.c.sigma = (t == 0) ? 0.f : expf(0.5f * h->sched[DSX_SCH_POSTERIOR_LOG_VARIANCE_CLIPPED][t]);
+    DSX_TRY(run_step(h, g, j, 0, h->m.L, ha, s));
   }
   return DSX_OK;
 }
@@ -275,6 +270,13 @@ static void plms_coefs(const dsx_handle* h, int t, int interval, PlmsCoef& c) {
   c.a_diff = a_prev - a_t;
   c.kx = 1.0f / (a_t_sq * (a_t_sq + a_prev_sq));
   c.ke = 1.0f / (a_t_sq * (sqrtf((1.0f - a_prev) * a_t) + sqrtf((1.0f - a_t) * a_prev)));
+}
+
+// Linear multistep weights (shallow_diffusion_tts.py:188-197) of dsx_plms_update's `mode`: 0 = eps_t alone (the warm-up's
+// x'), 1 = (eps_t + eps'') / 2 (the warm-up's update), 2..4 = Adams-Bashforth over eps_t and the 1..3 previous eps.
+static void plms_weights(int mode, PlmsCoef& c) {
+  static const float w[5][5] = {{1, 0, 0, 0, 1}, {1, 1, 0, 0, 2}, {3, -1, 0, 0, 2}, {23, -16, 5, 0, 12}, {55, -59, 37, -9, 24}};
+  c.w0 = w[mode][0]; c.w1 = w[mode][1]; c.w2 = w[mode][2]; c.w3 = w[mode][3]; c.denom = w[mode][4];
 }
 
 static int sample_plms_impl(dsx_handle* h, float* x, const Geom& g, int t_start, int interval, cudaStream_t s) {
@@ -292,86 +294,39 @@ static int sample_plms_impl(dsx_handle* h, float* x, const Geom& g, int t_start,
   DSX_CUDA(cudaStreamSynchronize(s));
   DSX_TRY(launch_embed_table(h, h->ws.TVALS, n + 1, s));
   const dsx_strides xs = contiguous_mel(h->m.M, g.T);
-  float* E[5];
-  for (int i = 0; i < 5; ++i) E[i] = h->ws.EPS + static_cast<size_t>(i) * mel;
-  // history ring: hist[0] = most recent eps_t
-  float* hist[4] = {nullptr, nullptr, nullptr, nullptr};
-  int nh = 0, slot = 0;
-  const bool tc = h->precision != DSX_PREC_FP32_SIMT;
-  const DdpmCoef none{};
-  if (tc) {
-    // tcgen05 path: per evaluation the residual stack + ONE head kernel that also does the multistep combination, the
-    // get_x_pred update, the history store and the next evaluation's input projection (2 launches per PNDM step)
-    DSX_TRY(launch_tc_head(h, g, TC_INPROJ, x, xs, nullptr, nullptr, 0, 0, none, 0, 0, s));
-    for (int j = 0; j < n; ++j) {
-      const int t = steps[j];
-      float* e0 = E[slot];
-      PlmsFuse pf{};
-      plms_coefs(h, t, interval, pf.c);
-      const int next_flags = (j + 1 < n) ? TC_INPROJ : 0;
-      // residual stack of table row `row` followed by the head with `flags` / `pp` (fused into one launch where possible)
-      auto step = [&](int row, int flags, const PlmsFuse& pp, int next_row) -> int {
-        HeadArgs ha;
-        ha.flags = flags; ha.x = x; ha.xs = xs; ha.next_row0 = next_row; ha.row_per_b = 0; ha.plms = &pp;
-        bool head_done = false;
-        DSX_TRY(run_layers(h, g, row, 0, h->m.L, s, &ha, &head_done));
-        if (!head_done) DSX_TRY(launch_tc_head(h, g, flags, x, xs, nullptr, nullptr, 0, 0, none, next_row, 0, s, &pp));
-        return DSX_OK;
-      };
-      if (nh == 0) {
-        // x' = phi(x, eps_t, t) -> XTMP; eps'' = net(x', max(t - interval, 0)); eps* = (eps_t + eps'') / 2; x = phi(x, eps*, t)
-        PlmsFuse p1 = pf;
-        p1.c.w0 = 1.f; p1.c.denom = 1.f;
-        p1.eps_store = e0;
-        p1.x_out = h->ws.XTMP;
-        DSX_TRY(step(j, TC_HEAD | TC_PLMS | TC_INPROJ, p1, n));
-        pf.c.w0 = 1.f; pf.c.w1 = 1.f; pf.c.denom = 2.f;
-        pf.h1 = e0;
-        DSX_TRY(step(n, TC_HEAD | TC_PLMS | next_flags, pf, j + 1));
-      } else {
-        if (nh == 1) { pf.c.w0 = 3.f; pf.c.w1 = -1.f; pf.c.denom = 2.f; }
-        else if (nh == 2) { pf.c.w0 = 23.f; pf.c.w1 = -16.f; pf.c.w2 = 5.f; pf.c.denom = 12.f; }
-        else { pf.c.w0 = 55.f; pf.c.w1 = -59.f; pf.c.w2 = 37.f; pf.c.w3 = -9.f; pf.c.denom = 24.f; }
-        pf.h1 = hist[0];
-        pf.h2 = nh >= 2 ? hist[1] : nullptr;
-        pf.h3 = nh >= 3 ? hist[2] : nullptr;
-        pf.eps_store = e0;
-        DSX_TRY(step(j, TC_HEAD | TC_PLMS | next_flags, pf, j + 1));
-      }
-      hist[3] = hist[2]; hist[2] = hist[1]; hist[1] = hist[0]; hist[0] = e0;
-      nh = std::min(nh + 1, 4);
-      slot = (slot + 1) % 4;
-    }
-    return DSX_OK;
-  }
+  DSX_TRY(start_eval(h, g, x, xs, 0, 0, s));
+  // history ring of eps_t in ws.EPS slots 0..3: hist[0] = the most recent, nh of them filled
+  const float* hist[3] = {nullptr, nullptr, nullptr};
+  int nh = 0;
   for (int j = 0; j < n; ++j) {
-    const int t = steps[j];
-    float* e0 = E[slot];
-    DSX_TRY(run_eval(h, x, xs, g, j, 0, e0, s));
-    PlmsCoef c{};
-    plms_coefs(h, t, interval, c);
+    float* e0 = h->ws.EPS + static_cast<size_t>(j % 4) * mel;
+    const int next = (j + 1 < n) ? TC_INPROJ : 0;
+    PlmsFuse pf{};
+    plms_coefs(h, steps[j], interval, pf.c);
+    HeadArgs ha;
+    ha.x = x; ha.xs = xs; ha.plms = &pf;
     if (nh == 0) {
-      // x' = phi(x, eps_t, t); eps' = net(x', max(t - interval, 0)); eps* = (eps_t + eps') / 2
-      PlmsCoef c1 = c;
-      c1.w0 = 1.f; c1.denom = 1.f;
-      DSX_TRY(launch_plms_update(h, h->ws.XTMP, x, e0, nullptr, nullptr, nullptr, c1, mel, s));
-      float* e1 = E[4];
-      DSX_TRY(run_eval(h, h->ws.XTMP, xs, g, n, 0, e1, s));
-      c.w0 = 1.f; c.w1 = 1.f; c.denom = 2.f;
-      DSX_TRY(launch_plms_update(h, x, x, e0, e1, nullptr, nullptr, c, mel, s));
-    } else if (nh == 1) {
-      c.w0 = 3.f; c.w1 = -1.f; c.denom = 2.f;
-      DSX_TRY(launch_plms_update(h, x, x, e0, hist[0], nullptr, nullptr, c, mel, s));
-    } else if (nh == 2) {
-      c.w0 = 23.f; c.w1 = -16.f; c.w2 = 5.f; c.denom = 12.f;
-      DSX_TRY(launch_plms_update(h, x, x, e0, hist[0], hist[1], nullptr, c, mel, s));
+      // x' = phi(x, eps_t, t) -> XTMP; eps'' = net(x', max(t - interval, 0)); eps* = (eps_t + eps'') / 2; x = phi(x, eps*, t)
+      PlmsFuse p1 = pf;
+      plms_weights(0, p1.c);
+      p1.eps_store = e0; p1.x_out = h->ws.XTMP;
+      ha.flags = TC_HEAD | TC_PLMS | TC_INPROJ; ha.plms = &p1; ha.next_row0 = n;
+      DSX_TRY(run_step(h, g, j, 0, h->m.L, ha, s));
+      plms_weights(1, pf.c);
+      pf.h1 = e0;
+      ha.flags = TC_HEAD | TC_PLMS | next; ha.plms = &pf; ha.next_row0 = j + 1;
+      DSX_TRY(run_step(h, g, n, 0, h->m.L, ha, s));
     } else {
-      c.w0 = 55.f; c.w1 = -59.f; c.w2 = 37.f; c.w3 = -9.f; c.denom = 24.f;
-      DSX_TRY(launch_plms_update(h, x, x, e0, hist[0], hist[1], hist[2], c, mel, s));
+      plms_weights(nh + 1, pf.c);
+      pf.h1 = hist[0];
+      pf.h2 = nh >= 2 ? hist[1] : nullptr;
+      pf.h3 = nh >= 3 ? hist[2] : nullptr;
+      pf.eps_store = e0;
+      ha.flags = TC_HEAD | TC_PLMS | next; ha.next_row0 = j + 1;
+      DSX_TRY(run_step(h, g, j, 0, h->m.L, ha, s));
     }
-    hist[3] = hist[2]; hist[2] = hist[1]; hist[1] = hist[0]; hist[0] = e0;
-    nh = std::min(nh + 1, 4);
-    slot = (slot + 1) % 4;
+    hist[2] = hist[1]; hist[1] = hist[0]; hist[0] = e0;
+    nh = std::min(nh + 1, 3);
   }
   return DSX_OK;
 }
@@ -514,13 +469,7 @@ int dsx_plms_update(dsx_handle* h, float* x_out, const float* x_in, const float*
   DSX_CUDA(cudaSetDevice(h->device));
   PlmsCoef c{};
   plms_coefs(h, t, interval, c);
-  switch (mode) {
-    case 0: c.w0 = 1.f; c.denom = 1.f; break;
-    case 1: c.w0 = 1.f; c.w1 = 1.f; c.denom = 2.f; break;
-    case 2: c.w0 = 3.f; c.w1 = -1.f; c.denom = 2.f; break;
-    case 3: c.w0 = 23.f; c.w1 = -16.f; c.w2 = 5.f; c.denom = 12.f; break;
-    default: c.w0 = 55.f; c.w1 = -59.f; c.w2 = 37.f; c.w3 = -9.f; c.denom = 24.f; break;
-  }
+  plms_weights(mode, c);
   const size_t mel = static_cast<size_t>(B) * h->m.M * T;
   return launch_plms_update(h, x_out, x_in, eps[0], n_eps[mode] > 1 ? eps[1] : nullptr, n_eps[mode] > 2 ? eps[2] : nullptr,
                             n_eps[mode] > 3 ? eps[3] : nullptr, c, mel, s);

@@ -115,7 +115,6 @@ struct dsx_handle {
   bool loaded = false;
   int precision = DSX_PREC_FP32_SIMT;
   int tc_group = 1;
-  int use_graph = 0;
   int layer_limit = -1;
   int64_t launches = 0;
   int64_t stack_launches = 0;   // launches of k_tc_stack (dsx_stack.cu)
@@ -129,7 +128,6 @@ struct dsx_handle {
   CUtensorMap tm_w{}, tm_y[2][2]{}, tm_yh[2]{}, tm_ye[2]{}, tm_cond[2]{}, tm_s16[2]{}, tm_whead{}, tm_wsr{}, tm_wstk{}, tm_z{};
   CUtensorMap tm_y0s[2]{}, tm_zs[2]{}, tm_s16s[2][2]{}, tm_xst[2]{}, tm_y0st[2]{};   // stack kernel, [0]: 128 rows per CTA, [1]: 64 rows per CTA
   dsx::Geom tm_geom;           // geometry the activation maps were built for
-  int tm_group = 0;
   int profile = 0;
   void* stage[7] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};   // dsx_infer_host device staging
   size_t stage_cap[7] = {0, 0, 0, 0, 0, 0, 0};
@@ -165,8 +163,6 @@ struct dsx_handle {
   long long* trace_dev = nullptr;   // debug timeline buffer (dsx_debug_trace)
   std::vector<cudaEvent_t> prof_events;   // pairs (start, stop), prof_used of them recorded
   size_t prof_used = 0;
-  void* tm_base_y = nullptr;
-  void* tm_base_cond = nullptr;
 };
 
 namespace dsx {
@@ -175,8 +171,7 @@ namespace dsx {
 int simt_pack_model(dsx_handle* h, const dsx_diffnet_params* p, cudaStream_t s);
 int launch_embed_table(dsx_handle* h, const int64_t* t_dev, int rows, cudaStream_t s);
 int launch_pack_cond(dsx_handle* h, const float* cond, dsx_strides cs, const Geom& g, cudaStream_t s);
-int launch_inproj(dsx_handle* h, const float* x, dsx_strides xs, const Geom& g, int row0, int row_per_b,
-                  cudaStream_t s);
+int launch_inproj(dsx_handle* h, const float* x, dsx_strides xs, const Geom& g, cudaStream_t s);
 int launch_simt_layer(dsx_handle* h, int layer, const Geom& g, int row0, int row_per_b, cudaStream_t s);
 int launch_head(dsx_handle* h, const Geom& g, float* eps, cudaStream_t s);
 struct DdpmCoef { float A, Bc, c1, c2, sigma; };
@@ -196,8 +191,9 @@ int tc_pack_model(dsx_handle* h, cudaStream_t s);
 int tc_prepare_maps(dsx_handle* h, const Geom& g);
 int launch_tc_condproj(dsx_handle* h, const Geom& g, cudaStream_t s);
 int launch_tc_layers(dsx_handle* h, int l0, int l1, const Geom& g, int row0, int row_per_b, cudaStream_t s);
-// Head / tail of DiffNet on tensor cores.  flags: 1 = head (skip -> eps), 2 = write eps, 4 = DDPM update of x,
-// 8 = input projection of x (after the update if any) for the evaluation that uses table row (next_row0, row_per_b).
+// What follows the residual stack in a diffusion step: TC_HEAD = head (skip -> eps), TC_WRITE_EPS = write eps, TC_UPDATE = DDPM
+// update of x, TC_PLMS = PNDM update of x (PlmsFuse), TC_INPROJ = input projection of x (after the update if any) for the
+// evaluation that uses table row (next_row0, row_per_b).
 enum { TC_HEAD = 1, TC_WRITE_EPS = 2, TC_UPDATE = 4, TC_INPROJ = 8, TC_PLMS = 16 };
 // PNDM update fused into the head kernel (TC_PLMS): eps' = (w0 eps_t + w1 h1 + w2 h2 + w3 h3) / denom, x_out = phi(x, eps', t)
 // (usr/diff/shallow_diffusion_tts.py:174-199); eps_t is also stored to `eps_store` (history ring) when non-null.
@@ -209,18 +205,7 @@ struct PlmsFuse {
   float* eps_store;  // this evaluation's eps -> history ring slot (or null)
   float* x_out;      // result; null: in place
 };
-int launch_tc_head(dsx_handle* h, const Geom& g, int flags, float* x_state, dsx_strides xs, float* eps_out,
-                   const float* noise, uint64_t seed, uint64_t offset, DdpmCoef c, int next_row0, int row_per_b,
-                   cudaStream_t s, const PlmsFuse* plms = nullptr);
-bool tc_supported(const dsx_handle* h);
-int ensure_flags(dsx_handle* h, int n);
-int make_map_2d(CUtensorMap* m, const void* base, uint64_t rows, uint32_t box_rows);
-void reset_flags(dsx_handle* h);
-
-// ---- dsx_stack.cu ------------------------------------------------------------------------
-int tc_stack_pack(dsx_handle* h, cudaStream_t s);
-bool tc_stack_usable(dsx_handle* h, const Geom& g);
-// What follows the residual stack inside a diffusion step (k_tc_head's job), optionally fused into the stack launch
+// The same description serves the head fused into k_tc_stack, k_tc_head and the fp32 path's separate launches
 struct HeadArgs {
   int flags = 0;            // TC_* (0: no head)
   float* x = nullptr;       // mel state
@@ -232,6 +217,15 @@ struct HeadArgs {
   int next_row0 = 0, row_per_b = 0;   // FiLM table row of the NEXT evaluation (TC_INPROJ)
   const PlmsFuse* plms = nullptr;
 };
+int launch_tc_head(dsx_handle* h, const Geom& g, const HeadArgs& ha, cudaStream_t s);
+bool tc_supported(const dsx_handle* h);
+int ensure_flags(dsx_handle* h, int n);
+int make_map_2d(CUtensorMap* m, const void* base, uint64_t rows, uint32_t box_rows);
+void reset_flags(dsx_handle* h);
+
+// ---- dsx_stack.cu ------------------------------------------------------------------------
+int tc_stack_pack(dsx_handle* h, cudaStream_t s);
+bool tc_stack_usable(dsx_handle* h, const Geom& g);
 int launch_tc_stack(dsx_handle* h, int nl, const Geom& g, int row0, int row_per_b, int wset, cudaStream_t s,
                     const HeadArgs* head = nullptr);
 

@@ -13,6 +13,7 @@
 
 #include "dsx_internal.h"
 #include "dsx_rng.cuh"
+#include "dsx_update.cuh"
 
 namespace dsx {
 
@@ -211,13 +212,11 @@ int launch_pack_cond(dsx_handle* h, const float* cond, dsx_strides cs, const Geo
 }
 
 // ------------------------------------------------------------------------------------------
-// input projection (net.py:116-118): X[n][c] = relu(W_in[c][:] . x[b][:][t] + b_in[c]); for the
-// tcgen05 path also the first layer's conv input Y0 = fp16 split of (X + d_0).
+// input projection of the fp32 path (net.py:116-118): X[n][c] = relu(W_in[c][:] . x[b][:][t] + b_in[c]).  The tensor-core
+// paths project in k_tc_head / k_tc_stack.
 // ------------------------------------------------------------------------------------------
 constexpr int kInFrames = 16;
-__global__ void k_inproj(ModelDev m, const float* __restrict__ x, dsx_strides xs, int T, int Tp,
-                         float* __restrict__ X, __half* __restrict__ Y, size_t plane_elems,
-                         const float* __restrict__ dtab, int row0, int row_per_b) {
+__global__ void k_inproj(ModelDev m, const float* __restrict__ x, dsx_strides xs, int T, int Tp, float* __restrict__ X) {
   extern __shared__ float xt[];   // [kInFrames][M]
   const int b = blockIdx.y, t0 = blockIdx.x * kInFrames, M = m.M, C = m.C;
   for (int i = threadIdx.x; i < kInFrames * M; i += blockDim.x) {
@@ -226,7 +225,6 @@ __global__ void k_inproj(ModelDev m, const float* __restrict__ x, dsx_strides xs
     xt[f * M + mm] = (t < T) ? x[b * xs.b + mm * xs.c + t * xs.t] : 0.f;
   }
   __syncthreads();
-  const float* d0 = dtab ? dtab + static_cast<size_t>(row0 + b * row_per_b) * m.L * C : nullptr;
   for (int c = threadIdx.x; c < C; c += blockDim.x) {
     const float* w = m.in_w + static_cast<size_t>(c) * M;
     float acc[kInFrames];
@@ -242,26 +240,14 @@ __global__ void k_inproj(ModelDev m, const float* __restrict__ x, dsx_strides xs
     for (int f = 0; f < kInFrames; ++f) {
       int t = t0 + f;
       if (t >= T) continue;
-      float v = fmaxf(acc[f] + bias, 0.f);
-      size_t o = (static_cast<size_t>(b) * Tp + t) * C + c;
-      X[o] = v;
-      if (Y) {
-        float y = v + d0[c];
-        __half hi = __float2half_rn(y);
-        Y[o] = hi;
-        Y[plane_elems + o] = __float2half_rn(y - __half2float(hi));
-      }
+      X[(static_cast<size_t>(b) * Tp + t) * C + c] = fmaxf(acc[f] + bias, 0.f);
     }
   }
 }
 
-int launch_inproj(dsx_handle* h, const float* x, dsx_strides xs, const Geom& g, int row0, int row_per_b,
-                  cudaStream_t s) {
+int launch_inproj(dsx_handle* h, const float* x, dsx_strides xs, const Geom& g, cudaStream_t s) {
   dim3 grid((g.T + kInFrames - 1) / kInFrames, g.B);
-  const bool tc = h->precision != DSX_PREC_FP32_SIMT;
-  k_inproj<<<grid, 256, kInFrames * h->m.M * sizeof(float), s>>>(
-      h->m, x, xs, g.T, g.Tp, h->ws.X, tc ? h->ws.Y : nullptr, g.frames_padded() * h->m.C,
-      tc ? h->ws.DTAB : nullptr, row0, row_per_b);
+  k_inproj<<<grid, 256, kInFrames * h->m.M * sizeof(float), s>>>(h->m, x, xs, g.T, g.Tp, h->ws.X);
   h->launches++;
   DSX_CUDA(cudaGetLastError());
   return DSX_OK;
@@ -433,16 +419,12 @@ int launch_head(dsx_handle* h, const Geom& g, float* eps, cudaStream_t s) {
   return DSX_OK;
 }
 
-// p_sample after the network (shallow_diffusion_tts.py:134-166), same fp32 operation order
-// (no FMA contraction): x_recon = A*x - Bc*eps; clamp; mean = c1*x_recon + c2*x; + sigma*noise.
+// p_sample after the network (shallow_diffusion_tts.py:134-166, ddpm_step) with injected or Philox noise
 __global__ void k_ddpm_update(float* __restrict__ x, const float* __restrict__ eps, const float* __restrict__ noise,
                               uint64_t seed, uint64_t offset, DdpmCoef c, size_t n, int M, int T, int b_off) {
   size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x;
   if (i >= n) return;
-  float xv = x[i];
-  float xr = __fsub_rn(__fmul_rn(c.A, xv), __fmul_rn(c.Bc, eps[i]));
-  xr = fminf(fmaxf(xr, -1.f), 1.f);
-  float mean = __fadd_rn(__fmul_rn(c.c1, xr), __fmul_rn(c.c2, xv));
+  const float xv = x[i], ev = eps[i];
   float z = 0.f;
   if (c.sigma != 0.f) {
     if (noise) {
@@ -453,7 +435,7 @@ __global__ void k_ddpm_update(float* __restrict__ x, const float* __restrict__ e
       z = (m & 3) == 0 ? z4.x : (m & 3) == 1 ? z4.y : (m & 3) == 2 ? z4.z : z4.w;
     }
   }
-  x[i] = __fadd_rn(mean, __fmul_rn(c.sigma, z));
+  x[i] = ddpm_step(c, xv, ev, z);
 }
 
 int launch_ddpm_update(dsx_handle* h, float* x, const float* eps, const float* noise, uint64_t seed, uint64_t offset,
@@ -464,21 +446,13 @@ int launch_ddpm_update(dsx_handle* h, float* x, const float* eps, const float* n
   return DSX_OK;
 }
 
-// PLMS (shallow_diffusion_tts.py:174-199): eps' = (w0*e0 + w1*e1 + w2*e2 + w3*e3) / denom with the
-// reference's left-to-right fp32 order; x_out = x + a_diff * (kx*x - ke*eps')   (get_x_pred)
+// PLMS (shallow_diffusion_tts.py:174-199, plms_step) over e0 and the history e1..e3 that is given
 __global__ void k_plms_update(float* __restrict__ xo, const float* __restrict__ xi, const float* __restrict__ e0,
                               const float* __restrict__ e1, const float* __restrict__ e2,
                               const float* __restrict__ e3, PlmsCoef c, size_t n) {
   size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x;
   if (i >= n) return;
-  float comb = __fmul_rn(c.w0, e0[i]);
-  if (e1) comb = __fadd_rn(comb, __fmul_rn(c.w1, e1[i]));
-  if (e2) comb = __fadd_rn(comb, __fmul_rn(c.w2, e2[i]));
-  if (e3) comb = __fadd_rn(comb, __fmul_rn(c.w3, e3[i]));
-  float ep = __fdiv_rn(comb, c.denom);
-  float xv = xi[i];
-  float inner = __fsub_rn(__fmul_rn(c.kx, xv), __fmul_rn(c.ke, ep));
-  xo[i] = __fadd_rn(xv, __fmul_rn(c.a_diff, inner));
+  xo[i] = plms_step(c, xi[i], e0[i], e1 ? e1[i] : 0.f, e2 ? e2[i] : 0.f, e3 ? e3[i] : 0.f, e1, e2, e3);
 }
 
 int launch_plms_update(dsx_handle* h, float* x_out, const float* x_in, const float* e0, const float* e1,

@@ -54,6 +54,7 @@
 #include "dsx_ptx.cuh"
 #include "dsx_rng.cuh"
 #include "dsx_tc_common.cuh"
+#include "dsx_update.cuh"
 
 namespace dsx {
 
@@ -1008,27 +1009,18 @@ __global__ void __launch_bounds__(kThreads, 1) k_tc_stack(const __grid_constant_
             for (int i = 0; i < 4; ++i)
               if (row_valid) p.eps_out[eo + i * ec] = ev[i];
           }
-          if (upd) {                                          // p_sample, the reference's fp32 operation order
+          if (upd) {
 #pragma unroll
             for (int i = 0; i < 4; ++i) {
-              float xr = __fsub_rn(__fmul_rn(p.c.A, xv[i]), __fmul_rn(p.c.Bc, ev[i]));
-              xr = fminf(fmaxf(xr, -1.f), 1.f);
-              const float mean = __fadd_rn(__fmul_rn(p.c.c1, xr), __fmul_rn(p.c.c2, xv[i]));
-              xv[i] = __fadd_rn(mean, __fmul_rn(p.c.sigma, zn[i]));
+              xv[i] = ddpm_step(p.c, xv[i], ev[i], zn[i]);
               if (row_valid) xp[i * xc] = xv[i];
             }
           }
-          if (plms) {                                         // linear multistep combination + get_x_pred (k_plms_update)
+          if (plms) {
 #pragma unroll
             for (int i = 0; i < 4; ++i) {
               const size_t ei = eo + i * ec;
-              float comb = __fmul_rn(p.pl.c.w0, ev[i]);
-              if (hp[0]) comb = __fadd_rn(comb, __fmul_rn(p.pl.c.w1, hv[0][i]));
-              if (hp[1]) comb = __fadd_rn(comb, __fmul_rn(p.pl.c.w2, hv[1][i]));
-              if (hp[2]) comb = __fadd_rn(comb, __fmul_rn(p.pl.c.w3, hv[2][i]));
-              const float ep = __fdiv_rn(comb, p.pl.c.denom);
-              const float inner = __fsub_rn(__fmul_rn(p.pl.c.kx, xv[i]), __fmul_rn(p.pl.c.ke, ep));
-              xv[i] = __fadd_rn(xv[i], __fmul_rn(p.pl.c.a_diff, inner));
+              xv[i] = plms_step(p.pl.c, xv[i], ev[i], hv[0][i], hv[1][i], hv[2][i], hp[0], hp[1], hp[2]);
               if (row_valid) {
                 if (p.pl.eps_store) p.pl.eps_store[ei] = ev[i];
                 if (p.pl.x_out) p.pl.x_out[ei] = xv[i];

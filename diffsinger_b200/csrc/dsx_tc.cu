@@ -40,6 +40,7 @@
 #include "dsx_ptx.cuh"
 #include "dsx_rng.cuh"
 #include "dsx_tc_common.cuh"
+#include "dsx_update.cuh"
 
 namespace dsx {
 
@@ -1351,22 +1352,13 @@ __global__ void __launch_bounds__(kThreads, 1) k_tc_head(const __grid_constant__
           if (do_head) ev = __uint_as_float(e8[i]) + __ldg(p.bf + m);
           if ((p.flags & TC_WRITE_EPS) && row_valid) p.eps[(static_cast<size_t>(b) * p.M + m) * p.T + t] = ev;
           if (p.flags & TC_UPDATE) {
-            float xr = __fsub_rn(__fmul_rn(p.c.A, xv[i]), __fmul_rn(p.c.Bc, ev));
-            xr = fminf(fmaxf(xr, -1.f), 1.f);
-            const float mean = __fadd_rn(__fmul_rn(p.c.c1, xr), __fmul_rn(p.c.c2, xv[i]));
-            xv[i] = __fadd_rn(mean, __fmul_rn(p.c.sigma, zn[i]));
+            xv[i] = ddpm_step(p.c, xv[i], ev, zn[i]);
             if (row_valid) p.x[xrow + static_cast<size_t>(m) * p.xs.c] = xv[i];
           }
           if ((p.flags & TC_PLMS) && row_valid) {
-            // linear multistep combination + get_x_pred, the reference's left-to-right fp32 order (k_plms_update)
             const size_t ei = (static_cast<size_t>(b) * p.M + m) * p.T + t;
-            float comb = __fmul_rn(p.pl.c.w0, ev);
-            if (p.pl.h1) comb = __fadd_rn(comb, __fmul_rn(p.pl.c.w1, p.pl.h1[ei]));
-            if (p.pl.h2) comb = __fadd_rn(comb, __fmul_rn(p.pl.c.w2, p.pl.h2[ei]));
-            if (p.pl.h3) comb = __fadd_rn(comb, __fmul_rn(p.pl.c.w3, p.pl.h3[ei]));
-            const float ep = __fdiv_rn(comb, p.pl.c.denom);
-            const float inner = __fsub_rn(__fmul_rn(p.pl.c.kx, xv[i]), __fmul_rn(p.pl.c.ke, ep));
-            xv[i] = __fadd_rn(xv[i], __fmul_rn(p.pl.c.a_diff, inner));
+            xv[i] = plms_step(p.pl.c, xv[i], ev, p.pl.h1 ? p.pl.h1[ei] : 0.f, p.pl.h2 ? p.pl.h2[ei] : 0.f,
+                              p.pl.h3 ? p.pl.h3[ei] : 0.f, p.pl.h1, p.pl.h2, p.pl.h3);
             if (p.pl.eps_store) p.pl.eps_store[ei] = ev;
             if (p.pl.x_out) p.pl.x_out[ei] = xv[i];
             else p.x[xrow + static_cast<size_t>(m) * p.xs.c] = xv[i];
@@ -1604,7 +1596,7 @@ static int make_map_act(CUtensorMap* m, const void* base, int ch, int T, int Tp,
 
 int tc_prepare_maps(dsx_handle* h, const Geom& g) {
   const size_t plane = g.frames_padded() * kC;
-  if (h->tm_geom.B == g.B && h->tm_geom.T == g.T && h->tm_epoch == h->ws_epoch && h->tm_group == h->tc_group) return DSX_OK;
+  if (h->tm_geom.B == g.B && h->tm_geom.T == g.T && h->tm_epoch == h->ws_epoch) return DSX_OK;
   DSX_TRY(make_map_2d(&h->tm_w, h->m.wpack, static_cast<uint64_t>(h->m.L) * kRowsPerLayer, 128));
   for (int buf = 0; buf < 2; ++buf) {
     for (int pl = 0; pl < 2; ++pl)
@@ -1629,7 +1621,6 @@ int tc_prepare_maps(dsx_handle* h, const Geom& g) {
   }
   h->tm_geom = g;
   h->tm_epoch = h->ws_epoch;
-  h->tm_group = h->tc_group;
   return DSX_OK;
 }
 
@@ -1808,34 +1799,32 @@ static int launch_tc_head_t(dsx_handle* h, const TcHeadParams& prm, int tiles, c
   return DSX_OK;
 }
 
-int launch_tc_head(dsx_handle* h, const Geom& g, int flags, float* x_state, dsx_strides xs, float* eps_out,
-                   const float* noise, uint64_t seed, uint64_t offset, DdpmCoef c, int next_row0, int row_per_b,
-                   cudaStream_t s, const PlmsFuse* plms) {
+int launch_tc_head(dsx_handle* h, const Geom& g, const HeadArgs& ha, cudaStream_t s) {
   const ModelDev& m = h->m;
   TcHeadParams prm;
   memset(&prm, 0, sizeof(prm));
   prm.tm_s16[0] = h->tm_s16[0];
   prm.tm_s16[1] = h->tm_s16[1];
   prm.tm_wh = h->tm_whead;
-  prm.x = x_state;
-  prm.xs = xs;
-  prm.eps = eps_out;
-  prm.noise = noise;
-  prm.seed = seed;
+  prm.x = ha.x;
+  prm.xs = ha.xs;
+  prm.eps = ha.eps;
+  prm.noise = ha.noise;
+  prm.seed = ha.seed;
   prm.b_off = h->batch_offset;
-  prm.offset = offset;
-  prm.c = c;
-  if (plms) prm.pl = *plms;
+  prm.offset = ha.offset;
+  prm.c = ha.c;
+  if (ha.plms) prm.pl = *ha.plms;
   prm.X = h->ws.X;
   prm.Y = h->ws.Y;                       // layer 0 reads buffer 0
   prm.plane_elems = g.frames_padded() * kC;
   prm.bs = m.skip_b;
   prm.bf = m.fin_b;
   prm.bin = m.in_b;
-  prm.d0 = h->ws.DTAB + static_cast<size_t>(next_row0) * m.L * kC;
-  prm.d_row_stride = row_per_b * m.L * kC;
+  prm.d0 = h->ws.DTAB + static_cast<size_t>(ha.next_row0) * m.L * kC;
+  prm.d_row_stride = ha.row_per_b * m.L * kC;
   prm.T = g.T; prm.Tp = g.Tp; prm.tiles_per_utt = g.tiles_per_utt; prm.tiles = g.tiles; prm.B = g.B; prm.M = m.M;
-  prm.flags = flags;
+  prm.flags = ha.flags;
   prm.status = h->status_dev;
   prm.budget_ns = 2000000000ull;
   prm.trace = h->trace_dev;

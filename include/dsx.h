@@ -198,7 +198,8 @@ enum {
   DSX_OPT_CP_PREFETCH = 1,  /* tuning knob, results do not depend on it: 1 = the layer kernel's activation producer streams the
                                hoisted conditioner projection HBM -> L2 half a layer ahead of the gate epilogue */
   DSX_OPT_PROFILE = 2,      /* 1: bracket the residual-layer kernel(s) of every evaluation with CUDA events; 2: bracket the
-                               head / update kernel of every DDPM step instead; 0: off.  Setting it resets the sums */
+                               head / update kernel(s) of every evaluation instead (the head then runs as a launch of its
+                               own); 0: off.  Setting it resets the sums */
   DSX_OPT_STACK_MODE = 3,   /* 1 (default): all residual layers of an evaluation in ONE persistent launch whenever every
                                128-frame tile can own an SM at once (tiles <= co-resident CTAs); 0: one launch per layer */
   DSX_OPT_STACK_KERNEL = 4, /* 1 (default): the register-resident stack kernel (residual stream in registers, conv input in
